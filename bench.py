@@ -59,7 +59,29 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--reference-split", action="store_true",
                     help="N > 1: work on the reference's greedy edge-balanced split instead of the cost-balanced one")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the PageRank values the last timed step computed (what a caller of "
+                         "the timed path reads back; the reference arm: its sampled vertices) to DIR/pagerank_values.npy "
+                         "and their vertex ids to DIR/vertex_ids.npy")
     return ap.parse_args()
+
+
+DUMP_MAX_VERTICES = 4 << 20  # 4 B value + 8 B id each: 48 MiB at most
+
+
+def dump_outputs(path, values, vid=None):
+    """values[i] (float32) belongs to vertex vid[i] (default: i), stored as float64 ids (exact below 2^53).  Beyond
+    DUMP_MAX_VERTICES, a fixed, seeded sample of the positions is written (sorted; identical from run to run), so that two
+    builds run with the same arguments can be compared output for output."""
+    total = len(values)
+    vid = np.arange(total, dtype=np.int64) if vid is None else np.asarray(vid)
+    if total > DUMP_MAX_VERTICES:
+        keep = np.unique(np.random.default_rng(SEED).integers(0, total, DUMP_MAX_VERTICES))
+        values, vid = values[keep], vid[keep]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "pagerank_values.npy"), np.ascontiguousarray(values, np.float32))
+    np.save(os.path.join(path, "vertex_ids.npy"), vid.astype(np.float64))
+    return {"dir": path, "vertices_written": int(len(values)), "vertices_computed": int(total)}
 
 
 def load_peaks():
@@ -238,6 +260,7 @@ def main():
         for _ in range(args.warmup):
             step()
         times = [step() for _ in range(args.steps)]
+        dumped = dump_outputs(args.dump_outputs, out, blk["vid"]) if args.dump_outputs else None
         total = float(np.sum(times))
         mteps = edges * ITERS_PER_STEP * args.steps / total / 1e6
         sample = "%d iterations per step over %s" % (ITERS_PER_STEP, desc)
@@ -251,6 +274,8 @@ def main():
                 "gpu_launches": 0, "input_seconds": t_gen,
                 "note": "reference has no CPU compute path and needs Legion (SURVEY §8c): the oracle port is timed; "
                         "input generated by the oracle itself (libluxb is not loaded in this arm)"}
+        if dumped:
+            line["dump_outputs"] = dumped
         print(json.dumps(line))
         return 0
 
@@ -321,6 +346,13 @@ def main():
     total_launches = int(tsum[3])
     edges_total = ne * ITERS_PER_STEP * args.steps
     value = edges_total / dev_s_max / 1e6
+
+    dumped = None
+    if args.dump_outputs:
+        x_last = g.values()  # collective on several ranks
+        if rank == 0:
+            dumped = dump_outputs(args.dump_outputs, x_last)
+        del x_last
 
     # ---- end to end through the C ABI with host buffers (pinned): every rank moves ITS partition's values over PCIe
     # (luxb_set_local_values: H2D of the slice + device-side exchange; luxb_get_local_values: D2H of the slice), like
@@ -446,6 +478,8 @@ def main():
                 "roofline_whole_step": {"algorithmic_GBps_per_gpu": (8 * ne + 16 * nv) * ITERS_PER_STEP * args.steps
                                         / world / dev_s_max / 1e9, "frac": (8 * ne + 16 * nv) * ITERS_PER_STEP
                                         * args.steps / world / dev_s_max / 1e9 / peak}}
+        if dumped:
+            line["dump_outputs"] = dumped
         print(json.dumps(line))
     if dist is not None:
         dist.barrier()

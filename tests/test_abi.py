@@ -100,16 +100,15 @@ def test_write_lux_bytes_equal_the_oracle_writer(tmp_path):
 
 
 def test_convert_edgelist_matches_reference_converter(tmp_path):
-    """luxb_convert_edgelist vs tools/converter.cc built as is (oracle/_ref/converter): header, offsets and out-degree
-    trailer byte-identical, per-destination source multisets equal (the reference's std::sort by dst is unstable), and
-    byte-identical to the oracle's canonical writer."""
-    import subprocess
+    """luxb_convert_edgelist vs tools/converter.cc built as is (its output for this edge list is stored in
+    tests/golden/ref_converter.npz): header, offsets and out-degree trailer byte-identical, per-destination source
+    multisets equal (the reference's std::sort by dst is unstable), and byte-identical to the oracle's canonical writer."""
     import oracle as O
     import lux_b200 as L
-    rng = np.random.default_rng(2)
+    golden = np.load(os.path.join(ROOT, "tests", "golden", "ref_converter.npz"))
     nv, ne = 257, 5000
-    s = rng.integers(0, nv, ne).astype(np.uint32)
-    d = rng.integers(0, nv, ne).astype(np.uint32)
+    s, d = golden["n257_src"], golden["n257_dst"]
+    assert len(s) == len(d) == ne
     txt = tmp_path / "edges.txt"
     txt.write_text("".join("%d %d\n" % (a, b) for a, b in zip(s, d)))
     mine = str(tmp_path / "mine.lux")
@@ -119,19 +118,15 @@ def test_convert_edgelist_matches_reference_converter(tmp_path):
     O.lux_write(canon, row_end, src)
     a = open(mine, "rb").read()
     assert a == open(canon, "rb").read()
-    conv = os.path.join(ROOT, "oracle", "_ref", "converter")
-    if os.path.exists(conv):
-        ref = str(tmp_path / "ref.lux")
-        subprocess.check_call([conv, "-nv", str(nv), "-ne", str(ne), "-input", str(txt), "-output", ref], stdout=subprocess.DEVNULL)
-        b = open(ref, "rb").read()
-        hdr = 12 + 8 * nv
-        assert len(a) == len(b) and a[:hdr] == b[:hdr] and a[hdr + 4 * ne:] == b[hdr + 4 * ne:]
-        ra, rb = np.frombuffer(a[hdr:hdr + 4 * ne], np.uint32), np.frombuffer(b[hdr:hdr + 4 * ne], np.uint32)
-        lo = 0
-        for v in range(nv):
-            hi = int(row_end[v])
-            assert sorted(rb[lo:hi].tolist()) == ra[lo:hi].tolist()
-            lo = hi
+    b = golden["n257_lux"].tobytes()
+    hdr = 12 + 8 * nv
+    assert len(a) == len(b) and a[:hdr] == b[:hdr] and a[hdr + 4 * ne:] == b[hdr + 4 * ne:]
+    ra, rb = np.frombuffer(a[hdr:hdr + 4 * ne], np.uint32), np.frombuffer(b[hdr:hdr + 4 * ne], np.uint32)
+    lo = 0
+    for v in range(nv):
+        hi = int(row_end[v])
+        assert sorted(rb[lo:hi].tolist()) == ra[lo:hi].tolist()
+        lo = hi
     with pytest.raises(L.LuxError):
         L.convert_edgelist(str(txt), mine, nv, ne + 1)      # fewer edges in the file than announced
     with pytest.raises(L.LuxError):

@@ -336,28 +336,19 @@ def test_golden_vectors():
     assert np.array_equal(O.label_run(O.APP_SSSP, row_end, src, start=0)["active"], g["sssp0_active"])
 
 
-# ---- the real reference converter, when it has been built from /root/reference (oracle/build_ref.py) ----------
-_CONVERTER = os.path.join(os.path.dirname(GOLDEN), "..", "oracle", "_ref", "converter")
-
-
-@pytest.mark.skipif(not os.path.exists(_CONVERTER), reason="oracle/_ref/converter not built (needs /root/reference)")
+# ---- the real reference converter: tests/golden/ref_converter.npz holds edge lists and the bytes tools/converter.cc
+# (built as is by oracle/build_ref.py) wrote for them (tests/golden/make_golden.py) ----------------------------------
 def test_oracle_lux_writer_matches_reference_converter_binary(tmp_path):
     """tools/converter.cc run on an edge list must produce exactly what oracle.lux_write produces (the converter's
     std::sort by dst is unstable, so compare per-destination source MULTISETS plus every other byte)."""
-    import subprocess
-    rng = np.random.default_rng(1)
+    g = np.load(os.path.join(GOLDEN, "ref_converter.npz"))
     nv, ne = 300, 4000
-    s = rng.integers(0, nv, ne).astype(np.uint32)
-    d = rng.integers(0, nv, ne).astype(np.uint32)
-    txt = tmp_path / "edges.txt"
-    txt.write_text("".join("%d %d\n" % (a, b) for a, b in zip(s, d)))
-    out = str(tmp_path / "ref.lux")
-    subprocess.check_call([_CONVERTER, "-nv", str(nv), "-ne", str(ne), "-input", str(txt), "-output", out],
-                          stdout=subprocess.DEVNULL)
+    s, d = g["n300_src"], g["n300_dst"]
+    assert len(s) == len(d) == ne
     row_end, src = O.edges_to_csc(nv, s, d)
     mine = str(tmp_path / "mine.lux")
     O.lux_write(mine, row_end, src)
-    a, b = open(out, "rb").read(), open(mine, "rb").read()
+    a, b = g["n300_lux"].tobytes(), open(mine, "rb").read()
     assert len(a) == len(b)
     hdr = 12 + 8 * nv
     assert a[:hdr] == b[:hdr]                      # header + row_end
